@@ -2,7 +2,7 @@
 """Benchmark of the FlowNet2 forward hot path (BASELINE.json metric: frame-pairs/s, FlowNet2 forward
 @1024x436; correlation-layer HBM GB/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 ours:       one process per GPU; full FlowNet2 (CSS + SD + fusion) deploy net through the Caffe-surface
@@ -10,7 +10,8 @@ ours:       one process per GPU; full FlowNet2 (CSS + SD + fusion) deploy net th
             Weights are filled on rank 0 and sent with ONE NCCL broadcast of the parameter arena; every step
             ends with a gather of the flow fields to rank 0.  `value` times K steps with inputs resident in
             HBM; `e2e` times the same K steps with pinned-host inputs (H2D inside) and the flows read back
-            to the host (D2H inside).
+            to the host (D2H inside).  --dump-outputs DIR: rank 0 writes the flow fields of the last timed step as
+            DIR/predict_flow_final.npy; weights and inputs are seeded, so two builds can be compared output for output.
 reference:  the reference's own CPU forward on all host cores, ONE WHOLE 1024x436 pair per step (fixed workload, no
             scaling): oracle/_ref (the reference's layer sources compiled unmodified) runs conv/deconv (im2col +
             OpenBLAS sgemm), ReLU, Eltwise, Concat, FlowWarp, ChannelNorm; Correlation / Resample / DataAugmentation
@@ -50,7 +51,11 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 2 / config 3 / 448x320 / config 5 side measurements")
     ap.add_argument("--config5-only", action="store_true", help="print only the config 5 (FlowNet2-C training step) measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32)")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.config5_only):
+        ap.error("--dump-outputs writes the outputs of the forward path of --impl ours only")
+    return a
 
 
 def peaks():
@@ -60,6 +65,21 @@ def peaks():
         return {"hbm_gbs": d["hbm_gbs"], "bf16_tflops": d["bf16_tflops"], "bf16_tflops_sustained": d.get("bf16_tflops_sustained"),
                 "source": "measured (MEASURED_PEAKS.json)"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback (B200_PROFILING.md)"}
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def write_outputs(d, arrays):
+    """--dump-outputs: every array as d/<name>.npy, float32, DUMP_BYTES in all.  An array larger than its share is replaced by a
+    fixed, seeded sample of its flattened elements (in index order), the same sample for the same shape on every run."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096                  # room for the .npy header
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, np.float32)
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share // 4, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def config(args, n_gpus):
@@ -562,6 +582,9 @@ def run_ours(args):
         t_begin = time.time()
         ms = timed(step_device, args.steps, device_finish)
         t_end = time.time()
+        # the flow fields a caller of the timed path receives from its last step (on rank 0: every rank's, gathered)
+        last_flow = (flow_root if world > 1 else flow_out)[(dev_state["i"] - 1) & 1]
+        dumped = last_flow.cpu().numpy() if args.dump_outputs and rank == 0 else None
         clocks = clocks_sampler_stop(sampler, t_begin, t_end) if rank == 0 else None
         # graph replays do not go through the launch counter: count = kernels per forward + layout copies
         per_step_launches = net.launches_per_forward + 3
@@ -654,10 +677,10 @@ def run_ours(args):
         if world == 1 and not args.no_extra:
             del net
             torch.cuda.empty_cache()
-            line["extra"] = {"config2": side_config(torch, F, "FlowNet2-C", 448, 320, 8),
-                             "config3": side_config(torch, F, "FlowNet2-CSS", 768, 384, 4),
-                             "flownet2_448x320": side_config(torch, F, "FlowNet2", 448, 320, 4),
-                             "config5": train_config(torch, F)}
+            line["extra"] = {"config2": side_config(torch, F, "FlowNet2-C", 448, 320, 8, steps=args.steps),
+                             "config3": side_config(torch, F, "FlowNet2-CSS", 768, 384, 4, steps=args.steps),
+                             "flownet2_448x320": side_config(torch, F, "FlowNet2", 448, 320, 4, steps=args.steps),
+                             "config5": train_config(torch, F, steps=args.steps)}
             rg = reference_gpu_arm(args, B)
             if rg is not None:
                 line["extra"]["reference_gpu"] = rg
@@ -669,6 +692,8 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if dumped is not None:
+        write_outputs(args.dump_outputs, {"predict_flow_final": dumped})
     if line is not None:
         print(json.dumps(line), flush=True)
 

@@ -36,13 +36,14 @@ def available():
     return os.path.exists(LIB_PATH)
 
 
-def build():
-    """Compile oracle/_ref (needs /root/reference; on the GPU box the prebuilt library is used)."""
+def build(required=True):
+    """Compile oracle/_ref from the reference checkout named by FN2_REFERENCE (an already built library is kept when the
+    checkout is absent).  required=False: return None instead of raising when neither exists."""
     import importlib.util
     spec = importlib.util.spec_from_file_location("build_ref", os.path.join(_HERE, "ref_shim", "build_ref.py"))
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
-    return m.build()
+    return m.build(required=required)
 
 
 def _find_openblas():

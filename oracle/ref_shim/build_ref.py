@@ -91,10 +91,13 @@ def compile_one(args):
     return obj
 
 
-def build(force=False):
+def build(force=False, required=True):
+    """-> the library path; None when the reference checkout is not readable and required is False."""
     if not os.path.isdir(REF):
         if os.path.exists(LIB):
             return LIB          # GPU box: the prebuilt library travelled with the snapshot
+        if not required:
+            return None
         raise RuntimeError("reference checkout %s not present and no prebuilt %s" % (REF, LIB))
     os.makedirs(os.path.join(GEN, "caffe/proto"), exist_ok=True)
     os.makedirs(OBJ, exist_ok=True)

@@ -181,11 +181,41 @@ def case_inputs(name):
 
 
 # ---- whole nets ------------------------------------------------------------------------------------------------------
-# (model, width, height, batch): small enough for the CPU oracle in seconds; the BASELINE shapes are compared live on the
-# GPU box (tests/test_ref_gpu.py) against oracle/_ref and against the float64 oracle.
+# (model, width, height, batch): small enough for the CPU oracle in seconds; the BASELINE shapes below are compared on the
+# GPU (tests/test_ref_gpu.py) live against the float64 oracle and against the stored reference outputs.
 NET_CASES = {
     "S_128x96": ("FlowNet2-S", 128, 96, 1),
     "C_192x100": ("FlowNet2-C", 192, 100, 1),
     "CSS_128x128": ("FlowNet2-CSS", 128, 128, 1),
     "FN2_128x64": ("FlowNet2", 128, 64, 1),
 }
+
+
+# ---- BASELINE.json shapes ----------------------------------------------------------------------------------------------
+# Correlation d=21, k=1 (FlowNet2-C) at the feature maps of configs 2, 3, 4, and the three nets of those configs at batch 1.
+# tests/golden/make_baseline_golden.py stores the reference's outputs for them in ref_baseline_golden.npz, as an evenly spaced
+# sample of each flattened output (baseline_sample): the whole tensors would be 30-50 MB each.
+BASELINE_CORR_SHAPES = [(8, 256, 40, 56), (4, 256, 48, 96), (4, 256, 56, 128)]
+BASELINE_CORR_TEXT = ('name: "c" type: "Correlation" bottom: "a" bottom: "b" top: "t" correlation_param { pad: 20 kernel_size: 1 '
+                      'max_displacement: 20 stride_1: 1 stride_2: 2 }')
+BASELINE_NETS = [("FlowNet2-C", 448, 320), ("FlowNet2-CSS", 768, 384), ("FlowNet2", 1024, 436)]
+BASELINE_SAMPLES = {"corr": 4096, "net": 8192}
+
+
+def baseline_corr_inputs(shape):
+    r = np.random.default_rng(shape[0] * 1000 + shape[2])
+    return r.standard_normal(shape).astype(np.float32), r.standard_normal(shape).astype(np.float32)
+
+
+def baseline_corr_key(shape):
+    return "corr/%dx%dx%dx%d" % tuple(shape)
+
+
+def baseline_net_key(model, w, h):
+    return "net/%s_%dx%d" % (model, w, h)
+
+
+def baseline_sample(a, n):
+    """n evenly spaced elements of the flattened array (every channel and row is hit)."""
+    a = np.asarray(a).reshape(-1)
+    return a[(np.arange(n, dtype=np.int64) * a.size) // n]

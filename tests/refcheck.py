@@ -19,6 +19,7 @@ import ref_cases as RC  # noqa: E402
 from oracle import oracle as O  # noqa: E402
 
 GOLD = os.path.join(HERE, "golden", "ref_golden.npz")
+BASELINE_GOLD = os.path.join(HERE, "golden", "ref_baseline_golden.npz")        # tests/golden/make_baseline_golden.py
 
 # kind -> relative tolerance (of max |reference output|) for "same arithmetic, different rounding order"
 TOL = {"correlation": 6e-7, "correlation1d": 6e-7, "resample": 1.5e-6, "resample_cubic": 6e-6, "channel_norm": 4e-7, "flow_warp": 5e-7, "conv": 3e-6,

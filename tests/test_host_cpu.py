@@ -31,7 +31,9 @@ def test_library_exports_every_declared_symbol(fn2):
 
 def test_library_is_sm100a_only():
     import subprocess
-    out = subprocess.run(["cuobjdump", "--list-elf", os.path.join(ROOT, "flownet2_b200", "libfn2.so")],
+    from flownet2_b200 import build
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")       # the toolkit that built the library
+    out = subprocess.run([cuobjdump, "--list-elf", os.path.join(ROOT, "flownet2_b200", "libfn2.so")],
                          capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs

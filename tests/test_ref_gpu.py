@@ -2,15 +2,14 @@
 
 (1) CUDA kernels (through the C-ABI) vs tests/golden/ref_golden.npz -- vectors the reference's own layer code produced on a
     B200 (tests/golden/make_ref_golden.py; inputs regenerated from seeds, tests/golden/ref_cases.py).
-(2) At the BASELINE.json shapes, live: the engine vs the float64-accumulating CPU oracle with the north_star's STRICT 1e-4
-    max-abs on predict_flow_final, and vs the reference's layers run on this GPU (oracle/_ref/libref_caffe.so, which travels
-    with the repo; if it is absent the reference leg is skipped, the oracle leg is not).
+(2) At the BASELINE.json shapes: the engine vs the float64-accumulating CPU oracle (live) with the north_star's STRICT 1e-4
+    max-abs on predict_flow_final, and vs tests/golden/ref_baseline_golden.npz -- samples of what the reference's layers
+    computed on a B200 for the same seeded inputs (tests/golden/make_baseline_golden.py).
 """
 import numpy as np
 import pytest
 
 from oracle import oracle as O
-from oracle import ref as R
 from oracle.net import OracleNet, synth_weights, write_caffemodel
 from tests import refcheck as RCK
 from tests.refcheck import RC
@@ -29,6 +28,11 @@ def ops(fn2):
 @pytest.fixture(scope="module")
 def gold():
     return RCK.golden()
+
+
+@pytest.fixture(scope="module")
+def baseline_gold():
+    return np.load(RCK.BASELINE_GOLD)
 
 
 def dev(a, channels_last=False):
@@ -171,35 +175,24 @@ def test_small_nets_match_reference_vectors(fn2, gold, cname):
 # ---------------------------------------------------------------------------------------------------------------------
 # BASELINE.json shapes, live
 # ---------------------------------------------------------------------------------------------------------------------
-def _ref_gpu():
-    if not R.available():
-        return False
-    R.set_mode(True, 0)
-    return True
-
-
-@pytest.mark.parametrize("shape", [(8, 256, 40, 56), (4, 256, 48, 96), (4, 256, 56, 128)])
-def test_correlation_baseline_shapes(ops, shape):
+@pytest.mark.parametrize("shape", RC.BASELINE_CORR_SHAPES)
+def test_correlation_baseline_shapes(ops, baseline_gold, shape):
     """Correlation d=21, k=1 (FlowNet2-C) at the three feature-map shapes of BASELINE.json's configs 2, 3, 4."""
-    r = rng(shape[0] * 1000 + shape[2])
-    a = r.standard_normal(shape).astype(np.float32)
-    b = r.standard_normal(shape).astype(np.float32)
+    a, b = RC.baseline_corr_inputs(shape)
     got = host(ops.correlation(dev(a, True), dev(b, True), 20, 1, 20, 1, 2))
     want = O.correlation_fwd(a, b, 20, 1, 20, 1, 2, 0, exact_order=False)           # float64 accumulation
     assert maxabs(got, want) <= 1e-6, maxabs(got, want)
-    if _ref_gpu():
-        text = ('name: "c" type: "Correlation" bottom: "a" bottom: "b" top: "t" correlation_param { pad: 20 kernel_size: 1 '
-                'max_displacement: 20 stride_1: 1 stride_2: 2 }')
-        ref, = R.run_layer(text, [a, b])
-        assert maxabs(got, ref) <= 1e-6, maxabs(got, ref)
+    ref = baseline_gold[RC.baseline_corr_key(shape)]
+    sample = RC.baseline_sample(got, len(ref))
+    assert maxabs(sample, ref) <= 1e-6, maxabs(sample, ref)
 
 
-@pytest.mark.parametrize("model,w,h", [("FlowNet2-C", 448, 320), ("FlowNet2-CSS", 768, 384), ("FlowNet2", 1024, 436)])
-def test_nets_at_baseline_sizes_strict_1e4(fn2, model, w, h):
-    """BASELINE configs 2, 3, 4 at batch 1: engine vs the float64 oracle AND vs the reference's layers on this GPU, both with the
-    north_star's absolute 1e-4 on predict_flow_final (|flow| reaches 10-30 px with the synthetic weights)."""
+@pytest.mark.parametrize("model,w,h", RC.BASELINE_NETS)
+def test_nets_at_baseline_sizes_strict_1e4(fn2, baseline_gold, model, w, h):
+    """BASELINE configs 2, 3, 4 at batch 1: engine vs the float64 oracle AND vs the reference's layers on a B200 (stored sample),
+    both with the north_star's absolute 1e-4 on predict_flow_final (|flow| reaches 10-30 px with the synthetic weights)."""
     proto = fn2.fill_template(fn2.model_template(model), w, h)
-    weights, blob = synth_weights(fn2.fill_template(fn2.model_template(model), 64, 64), 1701, proto)
+    _, blob = synth_weights(fn2.fill_template(fn2.model_template(model), 64, 64), 1701, proto)
     img0, img1 = smooth_images(rng(1701), 1, h, w)
     net = fn2.Net(proto, blob, fn2.TEST, batch=1)
     got = net.forward(img0=img0, img1=img1)["predict_flow_final"].copy()
@@ -210,7 +203,6 @@ def test_nets_at_baseline_sizes_strict_1e4(fn2, model, w, h):
     want = OracleNet(proto, blob, batch=1, f64acc=True).forward(img0=img0, img1=img1)["predict_flow_final"]
     assert np.abs(want).max() > 1.0, "degenerate: flow ~ 0"
     assert maxabs(got, want) <= 1e-4, ("engine vs float64 oracle", maxabs(got, want), float(np.abs(want).max()))
-    if _ref_gpu():
-        rnet = R.RefNet(proto, weights, batch=1)
-        ref = rnet.forward(img0=img0, img1=img1).blob("predict_flow_final")
-        assert maxabs(got, ref) <= 1e-4, ("engine vs reference GPU", maxabs(got, ref))
+    ref = baseline_gold[RC.baseline_net_key(model, w, h)]
+    sample = RC.baseline_sample(got, len(ref))
+    assert maxabs(sample, ref) <= 1e-4, ("engine vs reference GPU", maxabs(sample, ref))
