@@ -1,6 +1,8 @@
 // Shared device/host helpers for libfn2.so kernels (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
+#include <mutex>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -81,6 +83,21 @@ inline int num_sms() {
         if (sms <= 0) sms = 148;
     }
     return sms;
+}
+// cuTensorMapEncodeTiled, looked up once from the driver (the runtime API has no wrapper); nullptr if the driver lacks it.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline EncodeTiledFn encode_tiled_fn() {
+    static EncodeTiledFn fn = nullptr;
+    static std::once_flag once;
+    std::call_once(once, [] {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            fn = (EncodeTiledFn)p;
+    });
+    return fn;
 }
 // Grid for grid-stride elementwise kernels: enough CTAs to cover, capped at a multiple of the
 // SM count (148 SMs x 8 resident 256-thread CTAs).

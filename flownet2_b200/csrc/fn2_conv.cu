@@ -733,7 +733,7 @@ int fn2_conv_forward(const fn2_conv_desc* d, const fn2_tensor* bottom, const flo
         if (C4 <= 8) {
             const int grid = (int)min((long long)num_sms() * 8, (M + 255) / 256);
 #define FN2_PF_THREAD(C)                                                                                                   \
-            case C: if (k3 && d->pad_h == 1 && d->pad_w == 1 && !getenv("FN2_PF_NOTILE")) {                                \
+            case C: if (k3 && d->pad_h == 1 && d->pad_w == 1) {                                                            \
                         const size_t tsm = smem + (size_t)10 * 34 * (C + 1) * sizeof(float4);                               \
                         const int tgrid = (int)min((long long)num_sms() * 4, (long long)p.N * ((p.Wo + 31) / 32) * ((p.Ho + 7) / 8)); \
                         if (tsm > 48 * 1024) FN2_CUDA(cudaFuncSetAttribute(conv_pf3_tile_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm)); \

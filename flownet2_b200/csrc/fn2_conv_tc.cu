@@ -22,7 +22,6 @@
 // allocator, warps 4-7 converters, warps 8-11 drain + epilogue.  Small-Ci inputs use kernel-row or tap-group packing of
 // the K blocks (tc_small_ci).  DESIGN.md section 3 has the measurements behind each of these choices.
 #include <cuda.h>
-#include <mutex>
 
 #include "fn2_common.cuh"
 #include "fn2_tc_ptx.cuh"
@@ -49,15 +48,13 @@ struct TcParams {
     // tail split: the tiles of the last, partial wave [tail_first, ntotal) are cut into tail_z K ranges each so that they
     // spread over all SMs (448 tiles on 148 SMs: 3 + 1/8 rounds instead of 4); their partials are summed by a fix-up kernel
     int tail_first, tail_z, ntotal;
-    int tail_fix;                                 // 1: the K range that finishes LAST sums the tail_z partial tiles itself (no fix-up launch)
-    int* tail_cnt;                                // arrival counters of the tail tiles (zeroed before the launch)
-    FastDiv d_ntiles_p, d_cotiles, d_tiles_x, d_tiles_y, d_splits, d_tail_z;
+    FastDiv d_ntiles, d_cotiles, d_tiles_x, d_tiles_y, d_splits, d_tail_z;
     // Correlation on the same pipeline (corr_tc_forward): a unit = (sample, parity plane, 128-pixel tile of map 0, block of
     // cbw x cbh halo pixels of map 1); D[pixel][halo pixel] = <a, b> over C channels; the epilogue keeps the band that
     // lies inside the (2R+1)^2 displacement window.  W tiles are halo-pixel tiles of the pre-split map 1.
     int corr, cR, cS, cD, cbw, cbh, cnx, cnt;
     float cscale;
-    int cl, ntiles, ntiles_p, cotiles, total;     // cluster size (W multicast); pixel tiles (real / padded to cl), Co tiles, all tiles
+    int ntiles, cotiles, total;                   // pixel tiles, Co tiles, all tiles
     float comp_a, comp_b;                         // RZ bias model: shrink(n MMAs) = comp_a + comp_b * n
     int gcs;                                      // tap-group packing for Ci <= 16: padded channels per tap (4/8/12/16), 0 = off
     // kernel-row packing for Ci <= 16 on a dense input (pixel stride == rcs floats, guard band around the blob): the kw taps
@@ -67,7 +64,6 @@ struct TcParams {
     // the unshifted map, range of 32-pixel K segments); D[big channel][small channel] = sum over the segments' pixels.
     // Maps with few channels (wg_G = 8 .. 64 rows per tap) put 128 / wg_G taps side by side in one 128-row tile (wg_TPT).
     int wg_S, wg_ST, wg_BT, wg_segs, wg_segs_x, wg_sx, wg_G, wg_TPT, wg_taps;
-    int dbg;                                      // FN2_TC_DBG bits: 1 skip MMAs, 2 skip conversion math, 4 skip drain loads, 8 skip TMA A
     short dy[49], dx[49], widx[49];
 };
 
@@ -132,7 +128,6 @@ struct TcTile {
     int n, u0, v0, co0, cls, tap0, ntaps, steps;
     int k0, split;                                // first K step of this unit, split index
     int slot;                                     // >= 0: raw partial sums go to workspace slot `slot` (tail split)
-    int tq;                                       // tail split: index of the tile among the tail tiles (slot / tail_z)
     bool valid;
 };
 // MODE (compile time, so that each instantiation's role loops stay small -- the all-in-one kernel had ~1900 SASS instructions in
@@ -181,23 +176,20 @@ __device__ __forceinline__ TcTile tc_decode_tile(const TcParams& p, int tile) {
         t.slot = tile - p.tail_first;
         int q;
         p.d_tail_z.divmod(t.slot, q, tseg);
-        t.tq = q;
         tile = p.tail_first + q;
     }
     if (p.splits > 1) { int q; p.d_splits.divmod(tile, q, t.split); tile = q; }   // splits of a tile run side by side (shared A tiles in L2)
     int pix, r, cot = 0;
-    p.d_ntiles_p.divmod(tile, r, pix);
+    p.d_ntiles.divmod(tile, r, pix);
     t.cls = 0;
     if (r) p.d_cotiles.divmod(r, t.cls, cot);
-    t.valid = pix < p.ntiles;
-    if (!t.valid) pix = 0;
     int tx, ty, q2;
     p.d_tiles_x.divmod(pix, q2, tx);
     p.d_tiles_y.divmod(q2, t.n, ty);
     t.u0 = ty * p.th; t.v0 = tx * p.tw;
     t.co0 = cot * NT;
     t.tap0 = p.cls_tap0[t.cls]; t.ntaps = p.cls_ntaps[t.cls];
-    if (t.u0 >= p.cls_Hu[t.cls] || t.v0 >= p.cls_Wu[t.cls]) t.valid = false;      // tile outside this (smaller) parity class
+    t.valid = t.u0 < p.cls_Hu[t.cls] && t.v0 < p.cls_Wu[t.cls];       // false: tile outside this (smaller) parity class
     const int gsz = MODE == TC_GROUP ? 32 / p.gcs : 1;
     t.steps = MODE == TC_ROW ? p.rsteps : (MODE == TC_GROUP ? (t.ntaps + gsz - 1) / gsz : t.ntaps * p.cblocks);
     t.k0 = 0;
@@ -220,7 +212,7 @@ __device__ __forceinline__ TcTile tc_decode_tile(const TcParams& p, int tile) {
 template <int NT, int MODE>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapW, const float* __restrict__ bias,
-               float* __restrict__ out, float* __restrict__ ws, const TcParams p, long long* __restrict__ prof) {
+               float* __restrict__ out, float* __restrict__ ws, const TcParams p) {
     using G = TcGeo<NT>;
     extern __shared__ __align__(1024) unsigned char smem[];
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + G::R * G::STAGE_BYTES);
@@ -237,18 +229,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
     // running, so that its CTAs take over SMs the moment ours exit and run their prologue (barrier init, TMEM allocation)
     // there; it blocks in griddepcontrol.wait (below, before its first global access) until this grid has completed.
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    // CTAs of one cluster (p.cl consecutive blockIdx.x) always work on tiles with the same co0 and parity class, so they
-    // read the same W tiles: with p.cl > 1 each loads 1/cl of the rows and multicasts it to the whole cluster.  In that
-    // mode every CTA runs the full pipeline even for a tile outside the image/class (loads are zero-filled, nothing is
-    // stored); with p.cl == 1 such tiles are skipped.
-    const uint32_t crank = p.cl > 1 ? cluster_ctarank() : 0u;
-    const uint16_t cmask = (uint16_t)((1u << p.cl) - 1u);
-    const int wrows = NT / p.cl;                   // W rows this CTA loads per tile
     const int gsz = MODE == TC_GROUP ? 32 / p.gcs : 1;   // taps per K block when packing
-    const bool skip_invalid = p.cl == 1;
 
     if (tid == 0) {
-        for (int s = 0; s < G::R; s++) { mbar_init(&full[s], 1); mbar_init(&a_ready[s], 128); mbar_init(&done[s], p.cl); }
+        for (int s = 0; s < G::R; s++) { mbar_init(&full[s], 1); mbar_init(&a_ready[s], 128); mbar_init(&done[s], 1); }
         for (int s = 0; s < 2; s++) { mbar_init(&acc_full[s], 1); mbar_init(&acc_free[s], 128); }
         mbar_init(x_free, 128);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -259,13 +243,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
     }
     fence_before();
     __syncthreads();
-    if (p.cl > 1) cluster_sync_all();             // peers' barriers are initialised before any multicast can signal them
     fence_after();
     const uint32_t tmem = *tmem_slot;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // no-op unless launched with programmatic stream serialization
-    long long w0 = 0, w1 = 0, w2 = 0;
-    const bool timed = prof != nullptr;
-    const long long t_start = clock64();
 
     if (warp < 4) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 40;" ::: "memory");
@@ -276,17 +256,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             int s = 0; uint32_t ph = 1u;                // ph: parity to wait on done[s]
             for (int tile = blockIdx.x; tile < p.total; tile += gridDim.x) {
                 const TcTile T = tc_decode_tile<NT, MODE>(p, tile);
-                if (!T.valid && skip_invalid) continue;
+                if (!T.valid) continue;
                 const int cx0 = T.v0 * p.su, cy0 = T.u0 * p.sv;
                 auto load_w = [&](unsigned char* st, uint64_t* bar, int c0, int blk) {
-                    unsigned char* wh = st + A_TILE_BYTES + crank * wrows * 128;
-                    if (p.cl > 1) {
-                        tma_load_4d_mc(wh, &mapW, bar, c0, T.co0 + crank * wrows, blk, 0, cmask);
-                        tma_load_4d_mc(wh + G::B_TILE_BYTES, &mapW, bar, c0, T.co0 + crank * wrows, blk, 1, cmask);
-                    } else {
-                        tma_load_4d(wh, &mapW, bar, c0, T.co0, blk, 0);
-                        tma_load_4d(wh + G::B_TILE_BYTES, &mapW, bar, c0, T.co0, blk, 1);
-                    }
+                    tma_load_4d(st + A_TILE_BYTES, &mapW, bar, c0, T.co0, blk, 0);
+                    tma_load_4d(st + A_TILE_BYTES + G::B_TILE_BYTES, &mapW, bar, c0, T.co0, blk, 1);
                 };
                 if constexpr (MODE == TC_CORR) {
                     const int py = T.cls / p.cS, px = T.cls % p.cS;
@@ -295,7 +269,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     const uint32_t bbytes = (uint32_t)(p.cbw * p.cbh * 128);
 #pragma unroll 1
                     for (int i = 0; i < T.steps; i++) {
-                        mbar_wait_t(&done[s], ph, &w0, timed);
+                        mbar_wait(&done[s], ph);
                         unsigned char* st = smem + (size_t)s * G::STAGE_BYTES;
                         mbar_expect_tx(&full[s], (uint32_t)A_TILE_BYTES + 2u * bbytes);
                         tma_load_4d(st, &mapA, &full[s], i * 32, ax, ay, T.n);
@@ -314,7 +288,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     const int tpt = p.wg_TPT, gbytes = p.wg_G * 128;
 #pragma unroll 1
                     for (int i = 0; i < T.steps; i++) {
-                        mbar_wait_t(&done[s], ph, &w0, timed);
+                        mbar_wait(&done[s], ph);
                         unsigned char* st = smem + (size_t)s * G::STAGE_BYTES;
                         mbar_expect_tx(&full[s], (uint32_t)G::STAGE_BYTES);
                         for (int j = 0; j < tpt; j++) {
@@ -333,7 +307,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     int r = 0, kb = 0;
 #pragma unroll 1
                     for (int i = 0; i < T.steps; i++) {
-                        mbar_wait_t(&done[s], ph, &w0, timed);
+                        mbar_wait(&done[s], ph);
                         unsigned char* st = smem + (size_t)s * G::STAGE_BYTES;
                         mbar_expect_tx(&full[s], (uint32_t)G::STAGE_BYTES);
                         tma_load_4d(st, &mapA, &full[s], kb * 32, T.v0, cy0 + p.dy[r * p.rkw], T.n);
@@ -345,7 +319,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     // several taps share one 32-wide K block: one small box {gcs channels, tw, th} per tap
                     const int box_bytes = 128 * gcs * 4;
                     for (int i = 0, t0 = 0; i < T.steps; i++, t0 += gsz) {
-                        mbar_wait_t(&done[s], ph, &w0, timed);
+                        mbar_wait(&done[s], ph);
                         unsigned char* st = smem + (size_t)s * G::STAGE_BYTES;
                         const int nt = min(gsz, T.ntaps - t0);
                         mbar_expect_tx(&full[s], (uint32_t)(nt * box_bytes + 2 * G::B_TILE_BYTES));
@@ -361,7 +335,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     int cx = cx0 + p.dx[t], cy = cy0 + p.dy[t], wi = p.widx[t];
 #pragma unroll 1
                     for (int i = 0; i < T.steps; i++) {
-                        mbar_wait_t(&done[s], ph, &w0, timed);
+                        mbar_wait(&done[s], ph);
                         unsigned char* st = smem + (size_t)s * G::STAGE_BYTES;
                         mbar_expect_tx(&full[s], (uint32_t)G::STAGE_BYTES);
                         tma_load_4d(st, &mapA, &full[s], cb * 32, cx, cy, T.n);
@@ -382,14 +356,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             uint32_t px = 1u;                           // parity to wait on x_free (one phase per tile)
             for (int tile = blockIdx.x; tile < p.total; tile += gridDim.x) {
                 const TcTile T = tc_decode_tile<NT, MODE>(p, tile);
-                if (!T.valid && skip_invalid) continue;
+                if (!T.valid) continue;
                 int in_chunk = 0;
-                if (G::SEPX && T.steps > 0) { mbar_wait_t(x_free, px, &w0, timed); px ^= 1u; }
+                if (G::SEPX && T.steps > 0) { mbar_wait(x_free, px); px ^= 1u; }
 #pragma unroll 1
                 for (int i = 0; i < T.steps; i++) {
-                    if (in_chunk == 0) mbar_wait_t(&acc_free[buf], pacc, &w0, timed);
-                    mbar_wait_t(&full[s], ph, &w1, timed);
-                    mbar_wait_t(&a_ready[s], ph, &w2, timed);
+                    if (in_chunk == 0) mbar_wait(&acc_free[buf], pacc);
+                    mbar_wait(&full[s], ph);
+                    mbar_wait(&a_ready[s], ph);
                     fence_after();
                     const uint32_t bh = su32(smem + (size_t)s * G::STAGE_BYTES + A_TILE_BYTES);
                     const uint64_t dbh0 = make_desc_sw128(bh), dbl0 = make_desc_sw128(bh + G::B_TILE_BYTES);
@@ -397,22 +371,19 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     const uint32_t d = tmem + (buf ? G::COL_HH1 : G::COL_HH0);
                     const bool chunk_end = (in_chunk == kd - 1) || (i == T.steps - 1);
                     if (elect_one()) {
-                        if (!(p.dbg & 1)) {
 #pragma unroll
-                            for (int kk = 0; kk < 4; kk++) {
-                                // +2 in the start-address field = +32 bytes = the next 8 TF32 columns of the swizzled tile
-                                if constexpr (G::WIDE) {
-                                    mma_tf32_ts(d, a_hi + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc_w, (in_chunk | kk) != 0);
-                                    mma_tf32_ts(d + NT, a_lo + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, 1);
-                                } else {
-                                    mma_tf32_ts(d, a_hi + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, (in_chunk | kk) != 0);
-                                    mma_tf32_ts(tmem + G::COL_X, a_hi + kk * 8, dbl0 + (uint64_t)(2 * kk), idesc, (i | kk) != 0);
-                                    mma_tf32_ts(tmem + G::COL_X, a_lo + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, 1);
-                                }
+                        for (int kk = 0; kk < 4; kk++) {
+                            // +2 in the start-address field = +32 bytes = the next 8 TF32 columns of the swizzled tile
+                            if constexpr (G::WIDE) {
+                                mma_tf32_ts(d, a_hi + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc_w, (in_chunk | kk) != 0);
+                                mma_tf32_ts(d + NT, a_lo + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, 1);
+                            } else {
+                                mma_tf32_ts(d, a_hi + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, (in_chunk | kk) != 0);
+                                mma_tf32_ts(tmem + G::COL_X, a_hi + kk * 8, dbl0 + (uint64_t)(2 * kk), idesc, (i | kk) != 0);
+                                mma_tf32_ts(tmem + G::COL_X, a_lo + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, 1);
                             }
                         }
-                        if (p.cl > 1) mma_commit_mc(&done[s], cmask);   // tell every CTA that multicasts into this stage
-                        else mma_commit(&done[s]);
+                        mma_commit(&done[s]);
                         if (chunk_end) mma_commit(&acc_full[buf]);
                     }
                     __syncwarp();
@@ -431,10 +402,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
         uint32_t ph = 0;                           // full[s] parity; done[s] is waited with ph ^ 1
         for (int tile = blockIdx.x; tile < p.total; tile += gridDim.x) {
             const TcTile T = tc_decode_tile<NT, MODE>(p, tile);
-            if (!T.valid && skip_invalid) continue;
+            if (!T.valid) continue;
 #pragma unroll 1
             for (int i = 0; i < T.steps; i++) {
-                mbar_wait_t(&full[s], ph, &w0, timed);
+                mbar_wait(&full[s], ph);
                 const float4* row = reinterpret_cast<const float4*>(smem + (size_t)s * G::STAGE_BYTES + m * 128);
                 uint32_t hi[32], lo[32];
                 float4 raw[8];
@@ -455,9 +426,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     else if (p.gcs == 8) gather_taps<8>(base, m, nt, hi, lo);
                     else if (p.gcs == 12) gather_taps<12>(base, m, nt, hi, lo);
                     else gather_taps<16>(base, m, nt, hi, lo);
-                } else if (p.dbg & 2) {
-#pragma unroll
-                    for (int j = 0; j < 32; j++) { hi[j] = 0x3f800000u; lo[j] = 0; }
                 } else if constexpr (MODE == TC_ROW) {
                     // row mode: taps that fall outside the image row (and the K padding) hold whatever follows in memory
                     const int x0 = (T.v0 + m % p.tw) * p.su - p.rpad;            // input column of tap 0
@@ -488,8 +456,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                     }
                 }
                 // the MMAs that read this A slot NSLOTS steps ago must have retired
-                if (s >= G::NSLOTS) mbar_wait_t(&done[s - G::NSLOTS], ph, &w1, timed);
-                else mbar_wait_t(&done[s - G::NSLOTS + G::R], ph ^ 1u, &w1, timed);
+                if (s >= G::NSLOTS) mbar_wait(&done[s - G::NSLOTS], ph);
+                else mbar_wait(&done[s - G::NSLOTS + G::R], ph ^ 1u);
                 fence_after();
                 tmem_st32(lane_addr + G::COL_A + 64 * (s % G::NSLOTS), hi);
                 tmem_st32(lane_addr + G::COL_A + 64 * (s % G::NSLOTS) + 32, lo);
@@ -512,7 +480,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
         int buf = 0; uint32_t pfull = 0;           // pfull: parity to wait on acc_full[buf]
         for (int tile = blockIdx.x; tile < p.total; tile += gridDim.x) {
             const TcTile T = tc_decode_tile<NT, MODE>(p, tile);
-            if (!T.valid && skip_invalid) continue;
+            if (!T.valid) continue;
             float acc[NT];
 #pragma unroll
             for (int j = 0; j < NT; j++) acc[j] = 0.f;
@@ -522,11 +490,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                 const int nsteps = min(p.kd, T.steps - c * p.kd);
                 // mean RZ shrink of the accumulation chain of this chunk
                 const float comp = p.comp_a + p.comp_b * (float)(G::MMAS_PER_STEP * nsteps);
-                mbar_wait_t(&acc_full[buf], pfull, &w0, timed);
+                mbar_wait(&acc_full[buf], pfull);
                 fence_after();
                 const uint32_t src = lane_addr + (buf ? G::COL_HH1 : G::COL_HH0);
-                if (p.dbg & 4) {
-                } else if constexpr (NT == 128) {
+                if constexpr (NT == 128) {
 #pragma unroll
                     for (int j0 = 0; j0 < NT; j0 += 64) {
                         uint32_t v0[32], v1[32];
@@ -645,49 +612,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                 continue;
             }
             const int u = T.u0 + yy, v = T.v0 + xx;
-            if (MODE == TC_PLAIN && T.slot >= 0 && p.tail_fix) {
-                // tail split, fixed up in the kernel: every K range stores its raw partial tile; the range that arrives LAST (an
-                // atomic counter per tile) sums the tail_z partials in slot order -- the order does not depend on who is last -- and
-                // writes the finished tile.  bar.sync 1 = the 128 drain threads.
-                const bool live = T.valid && u < p.cls_Hu[T.cls] && v < p.cls_Wu[T.cls];
-                float* o = ws + ((long long)T.slot * 128 + m) * NT;
-#pragma unroll
-                for (int j = 0; j < NT; j += 4) *reinterpret_cast<float4*>(o + j) = make_float4(acc[j], acc[j + 1], acc[j + 2], acc[j + 3]);
-                __threadfence();
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                uint32_t* flag = tmem_slot + 1;
-                if (m == 0) {
-                    const int prev = atomicAdd(p.tail_cnt + T.tq, 1);
-                    const bool l = prev == p.tail_z - 1;
-                    if (l) p.tail_cnt[T.tq] = 0;                         // everybody has arrived: leave the counter ready for the next launch
-                    *flag = l ? 1u : 0u;
-                }
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                const bool last = *flag != 0;
-                asm volatile("bar.sync 1, 128;" ::: "memory");            // flag is rewritten by the next tail unit
-                if (last && live) {
-                    __threadfence();
-                    const int oy = u * p.ou + p.cls_oy0[T.cls], ox = v * p.ov + p.cls_ox0[T.cls];
-                    float* dst = out + T.n * p.out_sn + (long long)oy * p.out_sh + (long long)ox * p.out_sw + T.co0;
-                    const float* src = ws + ((long long)T.tq * p.tail_z * 128 + m) * NT;
-#pragma unroll 4
-                    for (int j = 0; j < NT; j += 4) {
-                        float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-                        for (int z = 0; z < p.tail_z; z++) {
-                            const float4 x = __ldcg(reinterpret_cast<const float4*>(src + (long long)z * 128 * NT + j));
-                            a.x += x.x; a.y += x.y; a.z += x.z; a.w += x.w;
-                        }
-                        float r[4] = {a.x, a.y, a.z, a.w};
-#pragma unroll
-                        for (int e = 0; e < 4; e++) {
-                            if (p.has_bias) r[e] += __ldg(bias + T.co0 + j + e);
-                            if (p.relu) r[e] = r[e] > 0 ? r[e] : r[e] * p.slope;
-                        }
-                        *reinterpret_cast<float4*>(dst + j) = make_float4(r[0], r[1], r[2], r[3]);
-                    }
-                }
-                continue;
-            }
             if (T.valid && u < p.cls_Hu[T.cls] && v < p.cls_Wu[T.cls]) {
                 const int oy = u * p.ou + p.cls_oy0[T.cls], ox = v * p.ov + p.cls_ox0[T.cls];
                 if (T.slot >= 0) {
@@ -718,14 +642,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             }
         }
     }
-    if (prof && blockIdx.x == gridDim.x / 2 && lane == 0 && (warp == 0 || warp == 1 || warp == 4 || warp == 8)) {
-        long long* o = prof + (warp == 0 ? 0 : warp == 1 ? 4 : warp == 4 ? 8 : 12);
-        o[0] = clock64() - t_start; o[1] = w0; o[2] = w1; o[3] = w2;
-    }
     fence_before();
     __syncthreads();
     if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
-    if (p.cl > 1) cluster_sync_all();             // no CTA leaves while a peer may still multicast into it / signal its barriers
 }
 
 // ---- weight packing: Caffe layout -> [hi|lo][tap][Co][Ci32] with the TF32 split -------------------------------------
@@ -848,56 +767,6 @@ __global__ void tc_tail_reduce_kernel(const float* __restrict__ ws, const float*
     }
 }
 
-// Arrival counters of the in-kernel tail fix-up: a pool of zeroed regions handed out round-robin per launch (captured launches keep
-// theirs).  Every launch leaves its counters at zero again (the last arriver resets them), so a region may be reused as soon as the
-// launch that had it has finished; with 256 regions that is 256 tail-split launches later.
-constexpr int TAIL_CNT_REGION = 1024, TAIL_CNT_REGIONS = 256;
-static int* tc_tail_counters() {
-    static int* pool = nullptr;
-    static std::mutex mu;
-    static unsigned next = 0;
-    std::lock_guard<std::mutex> lk(mu);
-    if (!pool) {
-        if (cudaMalloc(&pool, (size_t)TAIL_CNT_REGION * TAIL_CNT_REGIONS * sizeof(int)) != cudaSuccess) { pool = nullptr; return nullptr; }
-        cudaMemset(pool, 0, (size_t)TAIL_CNT_REGION * TAIL_CNT_REGIONS * sizeof(int));
-    }
-    return pool + (size_t)(next++ % TAIL_CNT_REGIONS) * TAIL_CNT_REGION;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn tc_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)p;
-    });
-    return fn;
-}
-
-// FN2_TC_DBG & 16: per-role wait-time profile of CTA (0,0,0), printed by fn2_tc_prof_dump()
-int tc_pdl_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("FN2_TC_PDL"); v = (e && e[0] == '0') ? 0 : 1; }
-    return v;
-}
-int tc_num_sms() {
-    static int n = 0;
-    if (!n) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); if (n <= 0) n = 148; }
-    return n;
-}
-
-long long* tc_prof_buffer() {
-    static long long* buf = nullptr;
-    static int on = -1;
-    if (on < 0) { const char* e = getenv("FN2_TC_DBG"); on = (e && (atoi(e) & 16)) ? 1 : 0; if (on) { cudaMalloc(&buf, 16 * sizeof(long long)); cudaMemset(buf, 0, 16 * sizeof(long long)); } }
-    return buf;
-}
-
 int tc_enabled() {
     static int v = -1;
     if (v < 0) {
@@ -905,6 +774,22 @@ int tc_enabled() {
         v = (e && e[0] == '0') ? 0 : 1;
     }
     return v;
+}
+
+// Accumulation chains of the conv forward and weight gradient (tiles of NT columns) and of the correlation (corr).  The
+// a_hi*w_hi product is chained in the tensor core over kd K steps (4 MMAs each) and then drained to FP32 registers: 24 (NT =
+// 128) or 16 MMAs per chain keep the end-to-end flow error equal to the FP32 SIMT engine's; the correlation chains a whole
+// unit (4 * C/32 MMAs).  The drain adds back the mean round-toward-zero loss of the chain, comp_a + comp_b * n for n MMAs
+// (tools/tc_probe.cu test3, tools/tc_calibrate2.py); a per-binade (ulp) model was measured too and is no better, and the
+// residual after removing the mean (~half the loss, growing linearly with n) is what bounds kd.
+// FN2_TC_KD (NT = 128, correlation) / FN2_TC_KDW (narrower tiles) override kd; FN2_TC_COMP=0 turns the compensation off.
+void tc_chain_model(TcParams& p, int NT, bool corr) {
+    p.kd = corr ? p.cblocks : (NT == 128 ? 6 : 4);
+    if (const char* e = getenv(NT == 128 ? "FN2_TC_KD" : "FN2_TC_KDW")) { const int v = atoi(e); if (v >= 1 && v <= 1024) p.kd = v; }
+    const char* nocomp = getenv("FN2_TC_COMP");
+    const bool off = nocomp && nocomp[0] == '0';
+    p.comp_a = off ? 0.f : RZ_COMP_A;
+    p.comp_b = off ? 0.f : RZ_COMP_B;
 }
 
 }  // namespace
@@ -916,13 +801,12 @@ struct TcSmallCi { int mode, cs, gs, ngroups, rblocks; };
 static TcSmallCi tc_small_ci(const fn2_conv_desc* d, int ci_stride) {
     TcSmallCi m = {0, 0, 0, 0, 0};
     if (d->deconv || d->ci > 16 || d->kh * d->kw < 2) return m;
-    if (getenv("FN2_TC_NOPACK")) return m;
     m.cs = (d->ci + 3) / 4 * 4;
     m.gs = 32 / m.cs;
     m.ngroups = (d->kh * d->kw + m.gs - 1) / m.gs;
     m.rblocks = (d->kw * m.cs + 31) / 32;
     m.mode = 1;
-    if (d->input_guard_bytes >= 512 && ci_stride == m.cs && d->kh * m.rblocks <= m.ngroups && !getenv("FN2_TC_NOROW")) m.mode = 2;
+    if (d->input_guard_bytes >= 512 && ci_stride == m.cs && d->kh * m.rblocks <= m.ngroups) m.mode = 2;
     return m;
 }
 
@@ -931,8 +815,7 @@ static TcSmallCi tc_small_ci(const fn2_conv_desc* d, int ci_stride) {
 // tail split plan for a layer with `tiles` tile units of `steps` K steps each: returns z (1 = off) and the first tail tile
 static int tc_tail_plan(long long tiles, int steps, int* first, int NT = 128) {
     *first = (int)tiles;
-    if (getenv("FN2_TC_NOTAIL")) return 1;
-    const int nsm = tc_num_sms();
+    const int nsm = num_sms();
     if (steps < 16) return 1;                       // (tiles <= nsm: everything is "tail" -- 112 tiles become 560 fifths on 148 SMs)
     const long long full = tiles / nsm * nsm, r = tiles - full;
     if (r == 0) return 1;
@@ -965,7 +848,6 @@ static void tc_layer_geometry(const fn2_conv_desc* d, int N, int Ho, int Wo, int
 }
 
 static int tc_split_plan(const fn2_conv_desc* d, int N, int Ho, int Wo) {
-    if (getenv("FN2_TC_NOSPLIT")) return 1;
     if (!d->deconv && d->ci <= 16) return 1;                       // small-Ci packing modes do not split
     if (d->co % 16) return 1;
     const int NT = (d->co % 128 == 0) ? 128 : (d->co % 64 == 0 ? 64 : (d->co % 32 == 0 ? 32 : 16));
@@ -977,7 +859,7 @@ static int tc_split_plan(const fn2_conv_desc* d, int N, int Ho, int Wo) {
     const long long tiles = (long long)N * ((Wu + tw - 1) / tw) * ((Hu + th - 1) / th) * (d->co / NT) * ncls;
     const int ntaps = d->deconv ? max(1, d->kh / sh) * max(1, d->kw / sw) : d->kh * d->kw;
     const int steps = ntaps * ((d->ci + 31) / 32);
-    const int nsm = tc_num_sms();
+    const int nsm = num_sms();
     if (tiles * 2 > nsm || steps < 32) return 1;
     int z = (int)(nsm / tiles);
     z = min(z, steps / 16);
@@ -1031,7 +913,7 @@ int conv_tc_eligible(const fn2_conv_desc* d, const T4& in, const T4& out) {
     if (d->stride_h > 2 || d->stride_w > 2) return 0;
     if (((uintptr_t)in.p & 15) || (in.sw & 3) || (in.sh & 3) || (in.sn & 3)) return 0;
     if (((uintptr_t)out.p & 15) || (out.sw & 3) || (out.sh & 3) || (out.sn & 3)) return 0;
-    if (!tc_encode_fn()) return 0;
+    if (!encode_tiled_fn()) return 0;
     return 1;
 }
 
@@ -1071,7 +953,7 @@ static inline int floordiv_i(int a, int b) { return (a >= 0) ? a / b : -((-a + b
 int conv_tc_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const float* bias, const T4& out, float* ws, size_t ws_floats,
                     cudaStream_t st) {
     if (conv_tn_applicable(d)) return conv_tn_forward(d, in, wp, bias, out, st);
-    EncodeTiledFn enc = tc_encode_fn();
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) { set_error("conv_tc: cuTensorMapEncodeTiled unavailable"); return FN2_ERR_CUDA; }
     const int NT = (d->co % 128 == 0) ? 128 : (d->co % 64 == 0 ? 64 : (d->co % 32 == 0 ? 32 : 16));
     const int cip = (d->ci + 31) / 32 * 32;
@@ -1083,25 +965,11 @@ int conv_tc_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const
     if (p.splits > 1 && (!ws || ws_floats < (size_t)p.splits * in.n * out.h * out.w * d->co)) p.splits = 1;
     p.out_sn = out.sn; p.out_sh = out.sh; p.out_sw = out.sw;
     p.relu = d->relu; p.has_bias = d->has_bias; p.slope = d->negative_slope;
-    p.kd = NT == 128 ? 6 : 4;                     // chains of 24 resp. 16 MMAs per chunk: end-to-end flow error == FP32 SIMT engine's
-    if (const char* e = getenv(NT == 128 ? "FN2_TC_KD" : "FN2_TC_KDW")) { const int v = atoi(e); if (v >= 1 && v <= 1024) p.kd = v; }
-    // mean round-toward-zero shrink of an n-MMA accumulation chain, measured by tools/tc_probe.cu (test3)
-    const char* nocomp = getenv("FN2_TC_COMP");
-    // tools/tc_calibrate2.py (B200, profiles/r01_tc_calibration.txt): mean relative loss of one chunk = comp_a + comp_b * n,
-    // n = MMAs chained into the chunk accumulator (4 per step: only the a_hi*w_hi product goes there).
-    // A per-binade (ulp) model was measured too and is no better; the residual after removing the mean is ~half the loss
-    // and grows linearly with n, which is what bounds kd.
-    p.comp_a = (nocomp && nocomp[0] == '0') ? 0.f : 2.0e-8f;
-    p.comp_b = (nocomp && nocomp[0] == '0') ? 0.f : 1.67e-8f;
-    if (const char* e = getenv("FN2_TC_COMP_A")) p.comp_a = (float)atof(e);
-    if (const char* e = getenv("FN2_TC_COMP_B")) p.comp_b = (float)atof(e);
-    { const char* e = getenv("FN2_TC_DBG"); p.dbg = e ? atoi(e) : 0; }
+    tc_chain_model(p, NT, false);
 
     const TcSmallCi sm = tc_small_ci(d, (int)in.sw);
     p.gcs = sm.mode == 1 ? sm.cs : 0;
     p.rowmode = sm.mode == 2; p.rcs = sm.cs; p.rblocks = sm.rblocks; p.rsteps = d->kh * sm.rblocks; p.rkw = d->kw; p.rpad = d->pad_w; p.rW = in.w;
-    { const char* e = getenv("FN2_TC_CL"); p.cl = e ? atoi(e) : 1; if (p.cl != 1 && p.cl != 2 && p.cl != 4) p.cl = 1; if (NT / p.cl < 8) p.cl = NT / 8; }
-    if (p.cl > 1) p.splits = 1;                   // cluster mates must walk the same K steps to share W tiles
     // weights: [2][taps][Co][cip]   (group mode: [2][groups][Co][32])
     CUtensorMap mapW;
     {
@@ -1109,7 +977,7 @@ int conv_tc_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const
         const int nblk = sm.mode == 2 ? p.rsteps : (sm.mode == 1 ? sm.ngroups : d->kh * d->kw);
         cuuint64_t dims[4] = {(cuuint64_t)kin, (cuuint64_t)d->co, (cuuint64_t)nblk, 2};
         cuuint64_t strides[3] = {(cuuint64_t)kin * 4, (cuuint64_t)kin * d->co * 4, (cuuint64_t)kin * d->co * nblk * 4};
-        cuuint32_t box[4] = {32, (cuuint32_t)(NT / p.cl), 1, 1};
+        cuuint32_t box[4] = {32, (cuuint32_t)NT, 1, 1};
         cuuint32_t es[4] = {1, 1, 1, 1};
         CUresult r = enc(&mapW, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void*)wp, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1143,38 +1011,28 @@ int conv_tc_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) { set_error("conv_tc: activation tensor map failed (%d)", (int)r); return FN2_ERR_CUDA; }
         p.ntiles = p.N * p.tiles_x * p.tiles_y;
-        p.ntiles_p = (p.ntiles + p.cl - 1) / p.cl * p.cl;
         p.cotiles = d->co / NT;
-        p.total = p.ntiles_p * p.cotiles * p.ncls * p.splits;
-        p.ntotal = p.total; p.tail_first = p.total; p.tail_z = 1; p.tail_fix = 0; p.tail_cnt = nullptr;
-        p.d_ntiles_p.init(p.ntiles_p); p.d_cotiles.init(p.cotiles); p.d_tiles_x.init(p.tiles_x); p.d_tiles_y.init(p.tiles_y);
+        p.total = p.ntiles * p.cotiles * p.ncls * p.splits;
+        p.ntotal = p.total; p.tail_first = p.total; p.tail_z = 1;
+        p.d_ntiles.init(p.ntiles); p.d_cotiles.init(p.cotiles); p.d_tiles_x.init(p.tiles_x); p.d_tiles_y.init(p.tiles_y);
         p.d_splits.init(max(1, p.splits)); p.d_tail_z.init(1);
-        if (p.splits == 1 && p.cl == 1 && !sm.mode && ws) {
+        if (p.splits == 1 && !sm.mode && ws) {
             int first = 0, steps_min = 1 << 30;
             for (int c = 0; c < p.ncls; c++) steps_min = min(steps_min, p.cls_ntaps[c] * p.cblocks);
             const int tz = tc_tail_plan(p.total, steps_min, &first, NT);
             if (tz > 1 && ws_floats >= (size_t)(p.total - first) * tz * 128 * NT) {
                 p.tail_first = first; p.tail_z = tz; p.d_tail_z.init(tz);
                 p.total = first + (p.ntotal - first) * tz;
-                // FN2_TC_TAILFIX=1: the last K range to arrive sums the partial tiles inside the kernel instead of a fix-up launch.
-                // Built and parity-tested, but measured SLOWER (FlowNet2 1024x436 b4: 16.55 vs 15.84 ms per step, 36 launches fewer):
-                // the last arriver's drain warps hold their SM's pipeline while they re-read tail_z tiles, whereas the separate kernel
-                // spreads that over all SMs and overlaps the next layer's prologue (PDL).  Off by default.
-                static const bool fix = getenv("FN2_TC_TAILFIX") != nullptr;
-                p.tail_cnt = (fix && p.ntotal - first <= TAIL_CNT_REGION) ? tc_tail_counters() : nullptr;
-                p.tail_fix = p.tail_cnt ? 1 : 0;
             }
         }
         cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)min(p.total, tc_num_sms() / p.cl * p.cl), 1, 1);
+        cfg.gridDim = dim3((unsigned)min(p.total, num_sms()), 1, 1);
         cfg.blockDim = dim3(TC_THREADS);
         cfg.stream = st;
-        cudaLaunchAttribute attr[2];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)p.cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[1].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr; cfg.numAttrs = tc_pdl_enabled() ? 2 : 1;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = attr; cfg.numAttrs = 1;
 #define FN2_TC_LAUNCH(NTV, MODEV)                                                                                       \
         {                                                                                                               \
             static bool attr_set = false;                                                                               \
@@ -1183,7 +1041,7 @@ int conv_tc_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const
                 attr_set = true;                                                                                        \
             }                                                                                                           \
             cfg.dynamicSmemBytes = TcGeo<NTV>::SMEM;                                                                    \
-            FN2_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<NTV, MODEV>, mapA, mapW, bias, out.p, ws, p, tc_prof_buffer())); \
+            FN2_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<NTV, MODEV>, mapA, mapW, bias, out.p, ws, p));                \
         }
 #define FN2_TC_LAUNCH_NT(MODEV)                                                                                         \
         if (NT == 128) FN2_TC_LAUNCH(128, MODEV)                                                                        \
@@ -1196,7 +1054,7 @@ int conv_tc_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const
 #undef FN2_TC_LAUNCH_NT
 #undef FN2_TC_LAUNCH
         FN2_LAUNCH_CHECK();
-        if (p.tail_z > 1 && !p.tail_fix) {
+        if (p.tail_z > 1) {
             const long long work = (long long)(p.ntotal - p.tail_first) * 128 * (NT / 4);
             if (NT == 128) tc_tail_reduce_kernel<128><<<ew_grid(work, 256), 256, 0, st>>>(ws, bias, out.p, p);
             else if (NT == 64) tc_tail_reduce_kernel<64><<<ew_grid(work, 256), 256, 0, st>>>(ws, bias, out.p, p);
@@ -1312,13 +1170,12 @@ static WgPlan wg_plan(const fn2_conv_desc* d, int N, int H, int W) {
     g.NT = g.Cs >= 128 ? 128 : (g.Cs >= 64 ? 64 : (g.Cs >= 32 ? 32 : 16));
     g.BT = (g.Cb + 127) / 128; g.ST = (g.Cs + g.NT - 1) / g.NT;
     g.G = 128;
-    if (g.Cb <= 64 && !getenv("FN2_WG_NOGROUP")) { g.G = 8; while (g.G < g.Cb) g.G *= 2; }
+    if (g.Cb <= 64) { g.G = 8; while (g.G < g.Cb) g.G *= 2; }
     g.TPT = 128 / g.G; g.TG = (g.taps + g.TPT - 1) / g.TPT;
     g.segs_x = (g.Ws + 31) / 32; g.segs = N * g.Hs * g.segs_x;
     const int base = g.TG * g.BT * g.ST;
-    int S = (3 * tc_num_sms() + base - 1) / base;
+    int S = (3 * num_sms() + base - 1) / base;
     S = max(1, min(S, g.segs / 8));
-    if (const char* e = getenv("FN2_WG_SPLITS")) { const int v = atoi(e); if (v >= 1) S = min(v, max(1, g.segs)); }
     g.S = S;
     g.Wq = (g.Wb + g.sx - 1) / g.sx + 3;          // + 3: room for the column delay of the 4 copies
     g.Wq_p = (g.Wq + 3) / 4 * 4; g.Ws_p = (g.Ws + 3) / 4 * 4;
@@ -1419,9 +1276,9 @@ __global__ void wg_reduce_kernel(const float* __restrict__ part, float* __restri
 }
 
 int conv_tc_wgrad_eligible(const fn2_conv_desc* d) {
-    if (!tc_enabled() || getenv("FN2_WGRAD_SIMT") || d->engine == 1) return 0;      // engine 1 = `engine: CAFFE`: exact-FP32 SIMT everywhere
+    if (!tc_enabled() || d->engine == 1) return 0;      // engine 1 = `engine: CAFFE`: exact-FP32 SIMT everywhere
     if (d->kh * d->kw > 49 || d->stride_w > 8 || d->stride_h > 8) return 0;
-    if (!tc_encode_fn()) return 0;
+    if (!encode_tiled_fn()) return 0;
     return 1;
 }
 size_t conv_tc_wgrad_workspace_floats(const fn2_conv_desc* d, int N, int H, int W) {
@@ -1431,7 +1288,7 @@ size_t conv_tc_wgrad_workspace_floats(const fn2_conv_desc* d, int N, int H, int 
 
 int conv_tc_wgrad(const fn2_conv_desc* d, const T4& bottom, const T4& top_diff, float* dw, float* db, int accumulate, float* ws,
                   size_t ws_floats, cudaStream_t st) {
-    EncodeTiledFn enc = tc_encode_fn();
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) { set_error("conv_tc_wgrad: cuTensorMapEncodeTiled unavailable"); return FN2_ERR_CUDA; }
     const WgPlan g = wg_plan(d, bottom.n, bottom.h, bottom.w);
     if (!ws || ws_floats < conv_tc_wgrad_workspace_floats(d, bottom.n, bottom.h, bottom.w)) { set_error("conv_tc_wgrad: workspace too small"); return FN2_ERR_WORKSPACE; }
@@ -1466,15 +1323,11 @@ int conv_tc_wgrad(const fn2_conv_desc* d, const T4& bottom, const T4& top_diff, 
     memset(&p, 0, sizeof(p));
     p.N = g.N; p.Co = g.Cs; p.cblocks = 1;
     p.Ho = g.Hs; p.Wo = g.Ws;
-    p.splits = 1; p.cl = 1; p.tail_z = 1; p.su = g.sx; p.sv = g.sy; p.ou = p.ov = 1; p.ncls = 1;
+    p.splits = 1; p.tail_z = 1; p.su = g.sx; p.sv = g.sy; p.ou = p.ov = 1; p.ncls = 1;
     p.tw = 128; p.th = 1; p.tiles_x = p.tiles_y = 1;
     p.wg_S = g.S; p.wg_ST = g.ST; p.wg_BT = g.BT; p.wg_segs = g.segs; p.wg_segs_x = g.segs_x; p.wg_sx = g.sx;
     p.wg_G = g.G; p.wg_TPT = g.TPT; p.wg_taps = g.taps;
-    p.kd = g.NT == 128 ? 6 : 4;
-    if (const char* e = getenv(g.NT == 128 ? "FN2_TC_KD" : "FN2_TC_KDW")) { const int v = atoi(e); if (v >= 1 && v <= 1024) p.kd = v; }
-    const char* nocomp = getenv("FN2_TC_COMP");
-    p.comp_a = (nocomp && nocomp[0] == '0') ? 0.f : 2.0e-8f;
-    p.comp_b = (nocomp && nocomp[0] == '0') ? 0.f : 1.67e-8f;
+    tc_chain_model(p, g.NT, false);
     for (int ky = 0; ky < d->kh; ky++)
         for (int kx = 0; kx < d->kw; kx++) {
             const int t = ky * d->kw + kx, q = kx - d->pad_w;
@@ -1504,13 +1357,9 @@ int conv_tc_wgrad(const fn2_conv_desc* d, const T4& bottom, const T4& top_diff, 
         if (r != CUDA_SUCCESS) { set_error("conv_tc_wgrad: small-map tensor map failed (%d)", (int)r); return FN2_ERR_CUDA; }
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)min(p.total, tc_num_sms()), 1, 1);
+    cfg.gridDim = dim3((unsigned)min(p.total, num_sms()), 1, 1);
     cfg.blockDim = dim3(TC_THREADS);
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
 #define FN2_WG_LAUNCH(NTV)                                                                                              \
     {                                                                                                                   \
         static bool attr_set = false;                                                                                   \
@@ -1519,7 +1368,7 @@ int conv_tc_wgrad(const fn2_conv_desc* d, const T4& bottom, const T4& top_diff, 
             attr_set = true;                                                                                            \
         }                                                                                                               \
         cfg.dynamicSmemBytes = TcGeo<NTV>::SMEM;                                                                        \
-        FN2_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<NTV, TC_WGRAD>, mapA, mapB, (const float*)nullptr, (float*)nullptr, part, p, tc_prof_buffer())); \
+        FN2_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<NTV, TC_WGRAD>, mapA, mapB, (const float*)nullptr, (float*)nullptr, part, p));                   \
     }
     if (g.NT == 128) FN2_WG_LAUNCH(128)
     else if (g.NT == 64) FN2_WG_LAUNCH(64)
@@ -1538,13 +1387,13 @@ int corr_tc_eligible(const T4& b0, const T4& b1, const T4& top, int md, int s2) 
     if (b0.c % 32 || b0.sc != 1 || b1.sc != 1 || top.sc != 1) return 0;
     if (((uintptr_t)b0.p & 15) || (b0.sw & 3) || (b0.sh & 3) || (b0.sn & 3)) return 0;
     if (((uintptr_t)b1.p & 15) || (b1.sw & 3) || (b1.sh & 3) || (b1.sn & 3)) return 0;
-    if (!tc_encode_fn()) return 0;
+    if (!encode_tiled_fn()) return 0;
     return 1;
 }
 size_t corr_tc_workspace_floats(int N, int C, int H, int W) { return (size_t)2 * N * H * W * C; }
 
 int corr_tc_forward(const T4& b0, const T4& b1, const T4& top, int md, int s2, float* ws, size_t ws_floats, cudaStream_t st) {
-    EncodeTiledFn enc = tc_encode_fn();
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) { set_error("corr_tc: cuTensorMapEncodeTiled unavailable"); return FN2_ERR_CUDA; }
     const int N = b0.n, C = b0.c, H = b0.h, W = b0.w, S = s2, R = md / s2;
     if (!ws || ws_floats < corr_tc_workspace_floats(N, C, H, W)) { set_error("corr_tc: workspace too small"); return FN2_ERR_WORKSPACE; }
@@ -1562,12 +1411,8 @@ int corr_tc_forward(const T4& b0, const T4& b1, const T4& top, int md, int s2, f
     p.N = N; p.Co = NT; p.cblocks = C / 32;
     p.Ho = H; p.Wo = W;
     p.out_sn = top.sn; p.out_sh = top.sh; p.out_sw = top.sw;
-    p.splits = 1; p.cl = 1; p.tail_z = 1; p.su = S; p.sv = S; p.ou = p.ov = 1; p.ncls = 1;
-    p.kd = p.cblocks;                                                     // one chunk per unit: chain of 4 * C/32 MMAs
-    if (const char* e = getenv("FN2_TC_KD")) { const int v = atoi(e); if (v >= 1 && v <= 1024) p.kd = v; }
-    const char* nocomp = getenv("FN2_TC_COMP");
-    p.comp_a = (nocomp && nocomp[0] == '0') ? 0.f : 2.0e-8f;
-    p.comp_b = (nocomp && nocomp[0] == '0') ? 0.f : 1.67e-8f;
+    p.splits = 1; p.tail_z = 1; p.su = S; p.sv = S; p.ou = p.ov = 1; p.ncls = 1;
+    tc_chain_model(p, NT, true);
     const int Ws = (W + S - 1) / S, Hs = (H + S - 1) / S;
     p.tiles_x = (Ws + p.tw - 1) / p.tw; p.tiles_y = (Hs + p.th - 1) / p.th;
     p.total = N * S * S * p.tiles_x * p.tiles_y * p.cnt;
@@ -1592,13 +1437,9 @@ int corr_tc_forward(const T4& b0, const T4& b1, const T4& top, int md, int s2, f
         if (r != CUDA_SUCCESS) { set_error("corr_tc: map-1 tensor map failed (%d)", (int)r); return FN2_ERR_CUDA; }
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)min(p.total, tc_num_sms()), 1, 1);
+    cfg.gridDim = dim3((unsigned)min(p.total, num_sms()), 1, 1);
     cfg.blockDim = dim3(TC_THREADS);
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
     const int smem_bytes = TcGeo<NT>::SMEM + 128 * CORR_TR_STRIDE * (int)sizeof(float);
     static bool attr_set = false;
     if (!attr_set) {
@@ -1606,19 +1447,9 @@ int corr_tc_forward(const T4& b0, const T4& b1, const T4& top, int md, int s2, f
         attr_set = true;
     }
     cfg.dynamicSmemBytes = smem_bytes;
-    FN2_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<NT, TC_CORR>, mapA, mapB, (const float*)nullptr, top.p, (float*)nullptr, p, tc_prof_buffer()));
+    FN2_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<NT, TC_CORR>, mapA, mapB, (const float*)nullptr, top.p, (float*)nullptr, p));
     FN2_LAUNCH_CHECK();
     return FN2_OK;
 }
 
 }  // namespace fn2
-
-extern "C" __attribute__((visibility("default"))) void fn2_tc_prof_dump(void) {
-    long long h[16];
-    long long* b = fn2::tc_prof_buffer();
-    if (!b) return;
-    cudaDeviceSynchronize();
-    cudaMemcpy(h, b, sizeof(h), cudaMemcpyDeviceToHost);
-    printf("tc prof (cycles) producer: total %lld wait_empty %lld | mma: total %lld wait_acc_free %lld wait_full %lld wait_a_ready %lld | converter: total %lld wait_full %lld wait_a_free %lld | drain: total %lld wait_acc_full %lld\n",
-           h[0], h[1], h[4], h[5], h[6], h[7], h[8], h[9], h[10], h[12], h[13]);
-}

@@ -25,7 +25,6 @@
 //   * Taps are cut into passes of <= 192 accumulator columns (tensor memory: 2 x 192 accumulator + 2 x 64 A-slot columns).
 // Warp roles, barrier rings and PDL as in fn2_conv_tc.cu.  Reference ops replaced: conv_layer.cu:8-23, deconv_layer.cu:8-23.
 #include <cuda.h>
-#include <mutex>
 
 #include "fn2_common.cuh"
 #include "fn2_tc_ptx.cuh"
@@ -58,7 +57,6 @@ struct TnParams {
     int ngmax;                                   // W tile rows in shared memory (max taps per pass * Co)
     int RA, RW, wres;                            // raw-A ring depth, W ring depth, 1 = all W stages resident in shared memory
     int total;                                   // units = N * nstrips * nseg
-    int dbg;                                     // FN2_TN_DBG bits (ablations, wrong results): 1 skip scatter, 2 skip write-out/zero, 4 skip MMAs, 8 skip conversion
     float comp;                                  // mean RZ shrink of the 12*cblocks-MMA chain
     int relu, has_bias;
     float slope;
@@ -213,7 +211,6 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                             if (elect_one()) {
 #pragma unroll
                                 for (int kk = 0; kk < 4; kk++) {
-                                    if (p.dbg & 4) break;
                                     mma_tf32_ts(d, a_hi + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, (cb | kk) != 0);
                                     mma_tf32_ts(d, a_hi + kk * 8, dbl0 + (uint64_t)(2 * kk), idesc, 1);
                                     mma_tf32_ts(d, a_lo + kk * 8, dbh0 + (uint64_t)(2 * kk), idesc, 1);
@@ -254,7 +251,6 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                 const uint32_t slot = lane_addr + TN_COL_A + 64 * (it & 1);
 #pragma unroll
                 for (int half = 0; half < 2; half++) {
-                    if (p.dbg & 8) break;
                     uint32_t hi[16], lo[16];
 #pragma unroll
                     for (int j = 0; j < 4; j++) {
@@ -293,8 +289,6 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             bv[0] = __ldg(bias + cb_); bv[1] = __ldg(bias + cb_ + 1); bv[2] = __ldg(bias + cb_ + 2); bv[3] = __ldg(bias + cb_ + 3);
         }
         int buf = 0; uint32_t pfull = 0;
-        long long tw_ = 0, ts_ = 0, tf_ = 0, tz_ = 0, tA_ = 0, tB_ = 0, tC_ = 0, tD_ = 0; int ntl_ = 0;      // FN2_TN_DBG & 16: cycles waiting / scattering / writing out / zeroing
-        const bool prof_ = (p.dbg & 16) != 0;
         for (int u = blockIdx.x; u < p.total; u += gridDim.x) {
             const TnUnit U = tn_decode(p, u);
             const int x_base = p.S * U.c0 + p.ox_min;                 // output column of ring column 0
@@ -307,22 +301,19 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                 const int touched_lo = i0 * p.S + p.oy_min;
                 const int yrel0 = it_ * p.S - p.oy_min;            // + oy[r]: row of this lane's contribution relative to touched_lo
                 for (int ps = 0; ps < p.npass; ps++) {
-                    long long c0_ = prof_ ? clock64() : 0;
                     mbar_wait(&acc_full[buf], pfull);
                     fence_after();
-                    long long c1_ = prof_ ? clock64() : 0;
-                    tw_ += c1_ - c0_;
                     const uint32_t src = lane_addr + (uint32_t)(buf * TN_ACC_COLS + h * CH);
                     // Taps of one kernel row land in the same output row, a few columns apart: taps whose column offsets differ
                     // by a multiple of S hit the column of a NEIGHBOURING lane's tap, so they are first summed across lanes with
                     // shuffles (lane L collects what belongs to its own column) and only one read-modify-write per group reaches
                     // shared memory.  Lanes whose neighbour lies outside the warp (= outside the tile row) produce an incomplete
                     // sum for a column outside the strip's complete range, which is never written out.
-                    const int ng = (p.dbg & 1) ? 0 : p.ngrp[ps];
+                    const int ng = p.ngrp[ps];
 #pragma unroll 1
                     for (int gi = 0; gi < ng; gi++) {
                         const int tl0 = p.grp[ps][gi].tl0, nrow = p.grp[ps][gi].nrow, oyr = p.grp[ps][gi].oyr;
-                        if (gi && !(p.dbg & 128)) tn_group_sync(h);   // the other 3 warps of this channel half may still add into the rows we now target
+                        if (gi) tn_group_sync(h);                      // the other 3 warps of this channel half may still add into the rows we now target
                         int ring = rb + yrel0 + oyr;
                         if (ring >= p.RR) ring -= p.RR;
                         float* rowp = obuf + ring * rowstride + col0;
@@ -336,13 +327,11 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                             float a0[8], a1[8];
                             uint32_t v0[8], v1[8], v2[8], v3[8];
                             const uint32_t tsrc = src + (uint32_t)(tl0 * CO + c0);
-                            const long long q0_ = prof_ ? clock64() : 0;
                             tmem_ld8(tsrc, v0);
                             if (nrow > 1) tmem_ld8(tsrc + CO, v1);
                             if (nrow > 2) tmem_ld8(tsrc + 2 * CO, v2);
                             if (nrow > 3) tmem_ld8(tsrc + 3 * CO, v3);
                             tmem_wait_ld();
-                            const long long q1_ = prof_ ? clock64() : 0;
 #define FN2_TN_COMP(x) fmaf(__uint_as_float(x), p.comp, __uint_as_float(x))
 #pragma unroll
                             for (int c = 0; c < 8; c++) a0[c] = FN2_TN_COMP(v0[c]);
@@ -374,7 +363,6 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                                 }
                             }
 #undef FN2_TN_COMP
-                            const long long q2_ = prof_ ? clock64() : 0;
                             // read-modify-write of 8 different channel planes: all loads first (the compiler must otherwise assume that
                             // the store of plane c aliases the load of plane c+1 and serialises 8 shared-memory round trips)
                             float* o = rowp + c0 * p.CW + ox0;
@@ -392,25 +380,22 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                                 for (int c = 0; c < 8; c++) o1[c * p.CW] = t_[c] + a1[c];
                             }
                             __syncwarp();
-                            if (prof_) { const long long q3_ = clock64(); tA_ += q1_ - q0_; tB_ += q2_ - q1_; tC_ += q3_ - q2_; }
                         }
                     }
                     fence_before();
                     mbar_arrive(&acc_free[buf]);
                     if (buf) pfull ^= 1u;
                     buf ^= 1;
-                    if (!(p.dbg & 128)) tn_group_sync(h);
-                    if (prof_) ts_ += clock64() - c1_;
+                    tn_group_sync(h);
                 }
-                long long c2_ = prof_ ? clock64() : 0;
                 // rows no later tile of this unit can touch: write them out (inside the segment / image) and clear them.  The two
                 // channel halves never meet in the ring, so each group of 4 warps flushes its own half on its own barrier.
                 const int hi_row = (k == U.ntiles - 1) ? (i0 + p.th - 1) * p.S + p.oy_max + 1 : (i0 + p.th) * p.S + p.oy_min;
                 if (k == 0) flush_lo = touched_lo;
                 const bool do_flush = (k == U.ntiles - 1) || (++since_flush == p.F);
-                const int lo_row = flush_lo;
-                if (do_flush) { since_flush = 0; flush_lo = hi_row; }
-                if (do_flush && !(p.dbg & 2)) {
+                if (do_flush) {
+                    const int lo_row = flush_lo;
+                    since_flush = 0; flush_lo = hi_row;
                     constexpr int CG = CH / 4;                 // float4 groups per pixel in this half
                     constexpr int XPI = 128 / CG;              // columns per iteration
                     const int d128 = dt & 127;
@@ -433,13 +418,8 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                             *reinterpret_cast<float4*>(dst + (long long)xi * p.out_sw) = make_float4(rv[0], rv[1], rv[2], rv[3]);
                         }
                     }
-                }
-                if (do_flush && !(p.dbg & 128)) tn_group_sync(h);
-                long long c3_ = prof_ ? clock64() : 0;
-                tf_ += c3_ - c2_;
-                if (do_flush && !(p.dbg & 2)) {
+                    tn_group_sync(h);
                     const int n4 = (CH * p.CW) >> 2;           // this half of a ring row, a multiple of 4 floats (CW even)
-                    const int d128 = dt & 127;
                     for (int y = lo_row; y < hi_row; y++) {
                         int ring = rb + (y - touched_lo);
                         if (ring >= p.RR) ring -= p.RR;
@@ -447,16 +427,12 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                         float4* z = reinterpret_cast<float4*>(obuf + ring * rowstride + h * CH * p.CW);
                         for (int e = d128; e < n4; e += 128) z[e] = make_float4(0.f, 0.f, 0.f, 0.f);
                     }
+                    tn_group_sync(h);
                 }
-                if (do_flush && !(p.dbg & 128)) tn_group_sync(h);
-                if (prof_) { tz_ += clock64() - c3_; ntl_++; }
                 rb += advance;
                 while (rb >= p.RR) rb -= p.RR;
             }
         }
-        if (prof_ && blockIdx.x == 1 && (tid == 256 || tid == 384))
-            printf("tn drain h=%d: %d tiles, per tile cycles: wait acc_full %lld, scatter %lld (tmem ld+wait %lld, comp+shuffle %lld, smem rmw %lld), write-out %lld, zero %lld\n", h, ntl_,
-                   tw_ / max(1, ntl_), ts_ / max(1, ntl_), tA_ / max(1, ntl_), tB_ / max(1, ntl_), tC_ / max(1, ntl_), tf_ / max(1, ntl_), tz_ / max(1, ntl_));
     }
     fence_before();
     __syncthreads();
@@ -466,21 +442,6 @@ conv_tn_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 
 
 // ---- host ---------------------------------------------------------------------------------------------------------------
-typedef CUresult (*TnEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-TnEncodeFn tn_encode_fn() {
-    static TnEncodeFn fn = nullptr;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = (TnEncodeFn)p;
-    });
-    return fn;
-}
-
 // packed weights: [hi|lo][pass * cblocks + cb][ngmax rows = (tap in pass, co)][32 channels of K block cb]
 __global__ void tn_pack_kernel(const float* __restrict__ w, float* __restrict__ wp, int Ci, int Co, int kh, int kw, int deconv,
                                int cblocks, int ngmax, TnParams p) {
@@ -590,21 +551,17 @@ static bool tn_layer_plan(const fn2_conv_desc* d, TnParams* p) {
     // a_hi*w_hi one, while slices beyond the last real channel add exact zeros and lose nothing.  Checked by the mean signed error
     // of tests/test_ops_gpu.py::test_conv_taps_on_n_engine (< 1e-7 of the output scale for Ci = 40 .. 162).
     const char* nocomp = getenv("FN2_TC_COMP");
-    float bm = 1.67e-8f;
-    if (const char* e = getenv("FN2_TN_COMP_B")) bm = (float)atof(e);
-    p->comp = (nocomp && nocomp[0] == '0') ? 0.f : (2.0e-8f + 3.f * bm * (float)((d->ci + 7) / 8));
+    p->comp = (nocomp && nocomp[0] == '0') ? 0.f : (RZ_COMP_A + 3.f * RZ_COMP_B * (float)((d->ci + 7) / 8));
     // shared memory: raw-A ring + W (resident if it all fits, else a ring of 2..3 stages) + barriers + output ring.  The ring is
     // flushed (written out + cleared, two barriers) every F tiles; a larger F needs (F-1) * th * S more ring rows.
     const int wstage = 2 * p->ngmax * 128;
     const int nwall = p->npass * p->cblocks;
-    int fmax = 4;
-    if (const char* e = getenv("FN2_TN_F")) fmax = max(1, min(8, atoi(e)));
-    for (int F = fmax; F >= 1; F--) {
+    for (int F = 4; F >= 1; F--) {
         p->F = F; p->RR = span + (F - 1) * p->th * p->S;
         const int ring = p->RR * d->co * p->CW * 4;
         const int budget = 227 * 1024 - ring - 1024 - 256;
         p->RA = 4;
-        if (!getenv("FN2_TN_NORES") && p->RA * TN_A_BYTES + nwall * wstage <= budget) { p->wres = 1; p->RW = 0; return true; }
+        if (p->RA * TN_A_BYTES + nwall * wstage <= budget) { p->wres = 1; p->RW = 0; return true; }
         p->wres = 0;
         p->RW = min(3, (budget - p->RA * TN_A_BYTES) / wstage);
         if (p->RW >= 3) return true;                 // a 2-deep W ring costs more than the rarer flush saves (measured)
@@ -650,12 +607,11 @@ int conv_tn_plan(const fn2_conv_desc* d, int N, int Ho, int Wo, int* out8) {
 }
 
 int conv_tn_forward(const fn2_conv_desc* d, const T4& in, const float* wp, const float* bias, const T4& out, cudaStream_t st) {
-    TnEncodeFn enc = tn_encode_fn();
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) { set_error("conv_tn: cuTensorMapEncodeTiled unavailable"); return FN2_ERR_CUDA; }
     TnParams p;
     if (!tn_layer_plan(d, &p)) { set_error("conv_tn: layer not eligible"); return FN2_ERR_INVALID; }
     p.N = in.n; p.Hin = in.h; p.Win = in.w; p.Ho = out.h; p.Wo = out.w;
-    { const char* e = getenv("FN2_TN_DBG"); p.dbg = e ? atoi(e) : 0; }
     p.relu = d->relu; p.has_bias = d->has_bias; p.slope = d->negative_slope;
     p.out_sn = out.sn; p.out_sh = out.sh; p.out_sw = out.sw;
     p.nstrips = (p.Wo - (p.S * p.cshift + p.xa) + p.S * p.stepx - 1) / (p.S * p.stepx);

@@ -295,7 +295,6 @@ __global__ void corr_shift_kernel(T4 td, float* __restrict__ gx, int R, int S) {
 }
 
 static bool corr_fast_ok(const T4& b0, const T4& b1, const T4& td, const T4& d0, const T4& d1, const CbP& p, int corr_type, int s2) {
-    if (getenv("FN2_CORR_BWD_SLOW")) return false;
     if (corr_type != 0 || !p.identity_g || p.D != CF_DW * CF_DW || s2 < 1 || s2 > 2 || p.reach_x != CF_R * s2 || p.C % 32) return false;
     const T4* ts[4] = {&b0, &b1, &d0, &d1};
     for (const T4* t : ts)

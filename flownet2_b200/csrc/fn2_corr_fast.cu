@@ -19,7 +19,6 @@
 //   * epilogue: divide by C (sumelems, :106-108) and store straight into the strided top view (NCHW for
 //     drop-in use, NHWC/concat view inside the engine).
 #include <cuda.h>
-#include <mutex>
 #include <unordered_map>
 
 #include "fn2_common.cuh"
@@ -249,25 +248,8 @@ __global__ void corr_rearrange_generic_kernel(T4 in, float* __restrict__ ws, int
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)p;
-    });
-    return fn;
-}
-
 int make_map(CUtensorMap* m, float* base, int Ws, int Hs, int C, int NP, int bw, int bh) {
-    EncodeTiledFn fn = encode_fn();
+    EncodeTiledFn fn = encode_tiled_fn();
     if (!fn) { set_error("cuTensorMapEncodeTiled is not available from the driver"); return FN2_ERR_CUDA; }
     cuuint64_t dims[4] = {(cuuint64_t)Ws, (cuuint64_t)Hs, (cuuint64_t)C, (cuuint64_t)NP};
     cuuint64_t strides[3] = {(cuuint64_t)Ws * 4, (cuuint64_t)Ws * Hs * 4, (cuuint64_t)Ws * Hs * C * 4};

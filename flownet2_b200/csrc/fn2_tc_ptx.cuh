@@ -6,6 +6,10 @@
 namespace fn2 {
 namespace {
 
+// Mean relative loss of a chain of n tensor-core MMAs accumulating into one FP32 accumulator, which the B200 rounds toward
+// zero: RZ_COMP_A + RZ_COMP_B * n (tools/tc_calibrate2.py on a B200, profiles/r01_tc_calibration.txt).
+constexpr float RZ_COMP_A = 2.0e-8f, RZ_COMP_B = 1.67e-8f;
+
 // division by a launch constant without the ~40-instruction integer divide (the tile decode is on the critical path of the
 // single-thread producer and MMA roles once per tile): q = (umulhi(n, mul) + n) >> shift for n < 2^31
 struct FastDiv {
@@ -39,25 +43,9 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         if (++spins > (1u << 24)) __trap();       // a lost arrival becomes a launch error, never a hang
     }
 }
-// instrumented wait: accumulates the cycles spent waiting into *acc (debug profiling, FN2_TC_DBG & 16)
-__device__ __forceinline__ void mbar_wait_t(uint64_t* bar, uint32_t parity, long long* acc, bool timed) {
-    if (!timed) { mbar_wait(bar, parity); return; }
-    const long long t0 = clock64();
-    mbar_wait(bar, parity);
-    *acc += clock64() - t0;
-}
 __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
     asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
                  ::"r"(su32(dst)), "l"(map), "r"(su32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-// the same box, delivered to the same shared-memory offset (and signalling the same barrier offset) of every CTA in cta_mask
-__device__ __forceinline__ void tma_load_4d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3, uint16_t cta_mask) {
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-                 ::"r"(su32(dst)), "l"(map), "r"(su32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
@@ -70,10 +58,6 @@ __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(su32(bar)) : "memory");
-}
-__device__ __forceinline__ void mma_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(su32(bar)), "h"(cta_mask) : "memory");
 }
 // D[tmem_c] (+)= A[tmem_a] * B[desc_b]^T, kind::tf32, A from tensor memory
 __device__ __forceinline__ void mma_tf32_ts(uint32_t tmem_c, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {

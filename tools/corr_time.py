@@ -26,6 +26,4 @@ for (N, H, W) in [(4, 56, 128), (8, 40, 56)]:
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 10
     by = 4.0 * N * H * W * (2 * 256 + 441); fl = 2.0 * 441 * 256 * N * H * W
-    from flownet2_b200 import lib
-    if hasattr(lib(), "fn2_tc_prof_dump") and os.environ.get("FN2_TC_DBG"): lib().fn2_tc_prof_dump()
     print("NOTC=%s (%d,256,%d,%d): %.3f ms  %.0f GB/s algorithmic  %.1f TFLOP/s" % (os.environ.get("FN2_CORR_NOTC", "0"), N, H, W, ms, by / ms / 1e6, fl / ms / 1e9), flush=True)

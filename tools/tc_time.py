@@ -31,5 +31,4 @@ for (N, Ci, H, W, Co, k, s, p) in [(4, 473, 56, 128, 256, 3, 1, 1), (4, 12, 448,
     steps = k * k * ((Ci + 31) // 32)
     tiles = N * ((Ho * Wo + 127) // 128) * max(1, Co // (128 if Co % 128 == 0 else 64 if Co % 64 == 0 else 32 if Co % 32 == 0 else 16))
     rounds = (tiles + 147) // 148
-    if hasattr(l, "fn2_tc_prof_dump"): l.fn2_tc_prof_dump()
-    print("DBG=%s %s: %.3f ms, %d tiles (%d rounds) x %d steps -> %.0f cycles/step @1.9GHz" % (os.environ.get("FN2_TC_DBG", "0"), (N, Ci, H, W, Co, k, s), ms, tiles, rounds, steps, ms * 1e-3 * 1.9e9 / rounds / steps), flush=True)
+    print("%s: %.3f ms, %d tiles (%d rounds) x %d steps -> %.0f cycles/step @1.9GHz" % ((N, Ci, H, W, Co, k, s), ms, tiles, rounds, steps, ms * 1e-3 * 1.9e9 / rounds / steps), flush=True)
